@@ -40,7 +40,6 @@ WORKLOAD = '3dmatch_shape_pair_register'
 N_RAW = 250_000               # raw points per scan -> ~50k voxels at 0.05 m
 SAMPLE_N_RAW = 8_000          # CPU sample: same generator, ~4k voxels per cloud
 SAMPLE_EXTENT = (1.5, 1.2, 1.0)
-REF_TIME_BUDGET_S = 240       # --impl reference: stop starting full-size pairs once this is exceeded (>= 1 runs)
 REF_MIN_N_RAW = 1500          # the reference arm's untimed warm-up sample
 VOXEL = 0.05
 POOL = 3                      # distinct pairs per rank, cycled over the steps
@@ -285,12 +284,23 @@ def stage_isolated_parity(dgr, pair_dev):
     return {'error': repr(e)}
 
 
+def dump_outputs(dirname, last, last_e2e=None):
+  """What the last timed step returned, as float64 .npy files: the 4x4 pose register() hands its caller and the
+  inlier weight sum behind the branch choice.  `last_e2e` is the last step of the host-buffer (`e2e`) loop."""
+  os.makedirs(dirname, exist_ok=True)
+  out = {'pose': last[0], 'weight_sum': [last[2].get('wsum', np.nan)]}
+  if last_e2e is not None:
+    out.update(pose_e2e=last_e2e[0], weight_sum_e2e=[last_e2e[2].get('wsum', np.nan)])
+  for name, a in out.items():
+    np.save(os.path.join(dirname, name + '.npy'), np.asarray(a, np.float64))
+  log(f'[bench] outputs of the last timed step: {", ".join(sorted(out))} -> {dirname}')
+
+
 def run_reference(args):
   """The reference's CPU implementation of the path (the oracle port: MinkowskiEngine is not installable
   offline, nothing of the reference compiles into oracle/_ref) on the SAME configuration as the B200 arm:
-  full-size pairs of the same generator and seeds.  One such pair is minutes of CPU, so the run executes as
-  many of the K steps as fit REF_TIME_BUDGET_S after the first (at least one) and says how many
-  (cpu_baseline.steps_executed); pairs/s is per executed full-size pair, nothing is extrapolated."""
+  full-size pairs of the same generator and seeds.  One such pair is minutes of CPU, so the arm's default is
+  one step; it registers exactly K pairs (cpu_baseline.steps_executed) and nothing is extrapolated."""
   rank = int(os.environ.get('RANK', '0'))
   if rank != 0:
     return
@@ -302,7 +312,6 @@ def run_reference(args):
   t_warm, _ = cpu_sample_time(state, 100, n_raw=REF_MIN_N_RAW)
   log(f'[bench] reference arm: warm-up sample {t_warm:.1f} s; timing full-size pairs')
   times, info, parity = [], {}, None
-  t_begin = time.perf_counter()
   for i in range(args.steps):
     xyz0, xyz1, _ = syn.room_pair(1000 * rank + (i % POOL), n_raw=N_RAW)
     t = time.perf_counter()
@@ -312,8 +321,8 @@ def run_reference(args):
     if i == 0:
       parity = fixture_parity(T)
     log(f'[bench] reference arm: pair {i} N0={info["n0"]} N1={info["n1"]} {times[-1]:.1f} s')
-    if time.perf_counter() - t_begin + times[-1] > REF_TIME_BUDGET_S:
-      break
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, (T, taps['branch'], {'wsum': taps['wsum']}))
   n_exec = len(times)
   dt = float(sum(times))
   val = n_exec / dt
@@ -456,6 +465,8 @@ def run_ours(args):
   t_end = time.time()
   thr1 = cgroup_throttled_ms()
   clocks = sampler.stop(t_start, t_end) if sampler else None
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, res['last'], res_e2e['last'])
   arena = [dgr.native_context(k).stats() for k in range(inflight)] if dgr._native_ok() else None
 
   prof_rows, serial_ms, stage_ms, n_prof = None, None, None, min(K, 20)
@@ -607,15 +618,23 @@ def main():
   ap.add_argument('--gpus', type=int, default=1)
   ap.add_argument('--steps', type=int, default=None,
                   help='timed steps (default 100 for the B200 arm: ~1.5 s per region, so that one ~0.3 s host stall '
-                       'of a shared box costs 10-20 %% instead of halving the number; 10 for --impl reference)')
+                       'of a shared box costs 10-20 %% instead of halving the number; 1 for --impl reference, '
+                       'where one full-size pair is minutes of CPU)')
   ap.add_argument('--warmup', type=int, default=3)
   ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
   ap.add_argument('--pairs', type=int, default=0,
                   help='BASELINE config 4: register this many pairs (seeds 0..pairs-1) round-robin over the ranks - '
                        'the same total at every N (strong scaling); 0 = the contract mode (K steps per rank, weak)')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='after the timed steps, write what the last timed step returned (pose, weight sum) as '
+                       'DIR/<name>.npy, so that two builds can be compared output for output')
   args = ap.parse_args()
+  if args.steps is not None and args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.steps is not None and args.pairs > 0:
+    ap.error('--steps and --pairs exclude each other: with --pairs every pair is one timed step')
   if args.steps is None:
-    args.steps = 10 if args.impl == 'reference' else 100
+    args.steps = 1 if args.impl == 'reference' else 100
   if args.impl == 'reference':
     run_reference(args)
   else:

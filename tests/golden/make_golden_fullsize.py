@@ -14,8 +14,9 @@ What is stored (everything else is re-derivable from these on the GPU box withou
   sha_*                      sha256 of sel0 / sel1 (int64), coords0 / coords1 / coords6 (int32) bytes
   feat{0,1}_rows, feat_step  every feat_step-th row of the oracle's FCGF features
   idx1                       the oracle's correspondences (int32 [N0])
-  knn_gap                    float32 [N0]: float64 relative gap between the best and the second-best
-                             squared distance (rows with a tiny gap may legitimately flip)
+  knn_safe, gap_safe         np.packbits of the rows whose float64 relative gap between the best and the
+                             second-best squared distance exceeds gap_safe (rows with a smaller gap may
+                             legitimately flip)
   logit                      float32 [N0] inlier logits of the oracle on ITS correspondences
   wsum, branch               the gate
   T_refined, refine_iters    pose after Procrustes + SE(3) refinement (before ICP)
@@ -42,6 +43,7 @@ from oracle import pipeline as op                           # noqa: E402
 from oracle.registration import feature_knn, inlier_weights, se3_refine   # noqa: E402
 
 FEAT_STEP = 16
+GAP_SAFE = 2e-3        # relative top-2 gap above which a 5e-5 feature perturbation cannot flip the arg-min
 
 
 def sha(a):
@@ -102,7 +104,8 @@ def run(config):
              sha_coords0=sha(c0.astype(np.int32)), sha_coords1=sha(c1.astype(np.int32)),
              sha_coords6=sha(c6.astype(np.int32)), feat_step=FEAT_STEP,
              feat0_rows=f0[::FEAT_STEP].numpy(), feat1_rows=f1[::FEAT_STEP].numpy(),
-             idx1=idx1.astype(np.int32), knn_gap=gap, logit=logit.reshape(-1).numpy().astype(np.float32),
+             idx1=idx1.astype(np.int32), gap_safe=GAP_SAFE, knn_safe=np.packbits(gap > GAP_SAFE),
+             logit=logit.reshape(-1).numpy().astype(np.float32),
              wsum=wsum, branch=branch, T_gt=T_gt)
   if branch == 'procrustes':
     R, t, info = timed('refine', lambda: se3_refine(p0, p1[idx1], w, 2 * vs))

@@ -1,7 +1,7 @@
 """CUDA path vs the CPU oracle AT THE BASELINE.json SIZES, through committed fixtures
 (tests/golden/fullsize_config{2,3}.npz, made by tests/golden/make_golden_fullsize.py: one oracle run
 of the bench's own seed-0 pair - 250k raw points, ~51k / ~40k voxels - and of the full KITTI-shape
-pair syn.lidar_pair(0)).  /root/reference and the minutes-long oracle run are not needed here.
+pair syn.lidar_pair(0)).  Neither the reference project nor the minutes-long oracle run is needed here.
 
 Bars (north_star): voxel selection / coordinates / 6-D coordinates bit-exact (sha256 of the arrays);
 features <= 5e-5; correspondences identical wherever the float64 top-2 gap exceeds the feature
@@ -22,7 +22,6 @@ from deepglobalregistration_b200 import synthetic as syn
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 FEAT_TOL = 5e-5
-GAP_SAFE = 2e-3        # relative top-2 gap above which a 5e-5 feature perturbation cannot flip the arg-min
 
 
 def sha(a):
@@ -81,13 +80,13 @@ def test_correspondences(run):
   oracle's criterion, oracle/registration.py::feature_knn) - every row of the full-size problem."""
   g = run.gold
   idx = run.idx1.cpu().numpy()
-  want, gap = g['idx1'], g['knn_gap']
-  safe = gap > GAP_SAFE
+  want, gap_safe = g['idx1'], float(g['gap_safe'])
+  safe = np.unpackbits(g['knn_safe'], count=len(want)).astype(bool)
   assert safe.mean() > 0.5
   bad = int((idx[safe] != want[safe]).sum())
   assert bad == 0, f'{bad} of {int(safe.sum())} unambiguous correspondences differ from the oracle'
   flips = int((idx != want).sum())
-  print(f'config {run.config}: {flips} of {len(idx)} correspondences differ, all inside the gap <= {GAP_SAFE} band '
+  print(f'config {run.config}: {flips} of {len(idx)} correspondences differ, all inside the gap <= {gap_safe} band '
         f'({int((~safe).sum())} rows)')
   A, B = run.F0.double(), run.F1.double()
   bn = (B * B).sum(1)

@@ -1,126 +1,79 @@
 """oracle/pipeline.py::register against the reference's OWN DeepGlobalRegistration.register():
-core/deep_global_registration.py, core/knn.py, core/registration.py, model/*.py, util/*.py are
-imported unmodified from /root/reference and run end to end on the CPU, with
+core/deep_global_registration.py, core/knn.py, core/registration.py, model/*.py, util/*.py run
+unmodified end to end on the CPU, with
 * MinkowskiEngine  -> oracle/me_cpu.py (sparse operators of oracle/sparse_ops.py),
-* open3d           -> the I/O stand-in of shims.py + registration_icp backed by oracle/icp.py.
+* open3d           -> the I/O stand-in of shims.py + registration_icp backed by oracle/icp.py,
+and what they returned is stored in tests/golden/reference_register.npz (tests/golden/make_golden_reference.py).
 The sparse operators and ICP are therefore the oracle's on both sides; what this pins is everything
 else the oracle restates by hand: the order of the stages, dtypes, voxelisation and re-flooring, the
 6-D coordinate assembly, feature types, the sigmoid / clip / weight-sum gate and its thresholds, the
-arguments handed to GlobalRegistration and to ICP.  Needs /root/reference: skipped elsewhere."""
+arguments handed to GlobalRegistration and to ICP."""
+import hashlib
+import json
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
-import torch
 
-from deepglobalregistration_b200 import shims
 from deepglobalregistration_b200 import synthetic as syn
-from oracle import icp as oicp
-from oracle import me_cpu
 from oracle import pipeline as op
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'core')), reason='reference tree not present')
-_REF_PACKAGES = ('model', 'core', 'util')
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_register.npz')
 
 
-@pytest.fixture
-def reference_dgr(monkeypatch):
-  """The reference's DeepGlobalRegistration class, importable on a CPU-only box."""
-  restore_me = me_cpu.install()
-  o3d = shims._open3d_stub()
-  o3d.pipelines = types.ModuleType('open3d.pipelines')
-  o3d.pipelines.registration = types.ModuleType('open3d.pipelines.registration')
+def sha(a):
+  return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
-  icp_calls = []
 
-  def registration_icp(source, target, max_correspondence_distance, init=np.eye(4), *a, **k):
-    icp_calls.append(dict(init=np.array(init), max_dist=max_correspondence_distance, n_source=len(source.points),
-                          n_target=len(target.points)))
-    T, info = oicp.icp_point_to_point(np.asarray(source.points), np.asarray(target.points),
-                                      max_correspondence_distance, init)
-    return types.SimpleNamespace(transformation=T, fitness=info['fitness'], inlier_rmse=info['inlier_rmse'])
-  o3d.pipelines.registration.registration_icp = registration_icp
-  saved = {k: sys.modules.get(k) for k in list(sys.modules)
-           if k == 'open3d' or k.startswith('open3d.') or k.split('.')[0] in _REF_PACKAGES}
-  for k in saved:
-    del sys.modules[k]
-  sys.modules['open3d'] = o3d
-  sys.path.insert(0, REF)
-  # the reference calls torch.load(config.weights) on a path that must exist; writing and re-reading the
-  # 1 GB synthetic checkpoint costs minutes of page-cache traffic, so the patched loader hands back the
-  # in-memory dict registered for that path (the file-level boundary is covered by the GPU tests)
-  real_load = torch.load
-  preloaded = {}
-  monkeypatch.setattr(torch, 'load', lambda f, *a, **k: preloaded[str(f)] if str(f) in preloaded
-                      else real_load(f, *a, **dict(k, weights_only=False)))
-  cwd = os.getcwd()
-  try:
-    from core.deep_global_registration import DeepGlobalRegistration
-    DeepGlobalRegistration.icp_calls = icp_calls          # what the reference handed to open3d
-    DeepGlobalRegistration.preloaded = preloaded
-    yield DeepGlobalRegistration
-  finally:
-    os.chdir(cwd)
-    sys.path.remove(REF)
-    for k in [k for k in sys.modules if k == 'open3d' or k.startswith('open3d.') or k.split('.')[0] in _REF_PACKAGES]:
-      del sys.modules[k]
-    sys.modules.update({k: v for k, v in saved.items() if v is not None})
-    restore_me()
+@pytest.fixture(scope='module')
+def gold():
+  return np.load(GOLD)
 
 
 @pytest.mark.parametrize('feature_type,dtype', [('ones', np.float64), ('coords', np.float32)])
-def test_reference_register_equals_oracle_pipeline(reference_dgr, tmp_path, feature_type, dtype, capsys):
+def test_reference_register_equals_oracle_pipeline(gold, feature_type, dtype):
+  ref = {k[len(f'reg_{feature_type}_'):]: gold[k] for k in gold.files if k.startswith(f'reg_{feature_type}_')}
   state = syn.make_checkpoint(1, inlier_feature_type=feature_type)
-  path = tmp_path / 'ckpt.pth'
-  path.write_bytes(b'')
-  reference_dgr.preloaded[str(path)] = state
   xyz0, xyz1, _ = syn.room_pair(7, n_raw=5000, extent=(1.2, 1.0, 0.8))
   xyz0, xyz1 = xyz0.astype(dtype), xyz1.astype(dtype)
-  cfg = types.SimpleNamespace(weights=str(path), clip_weight_thresh=0.05)
-  dgr = reference_dgr(cfg, device=torch.device('cpu'))
-  assert dgr.use_icp is True and dgr.voxel_size == state['config']['voxel_size']
-  # one run with the reference's default (use_icp = True); the pose it hands to open3d's ICP is tap A
-  T_ref = dgr.register(xyz0, xyz1)
+  # the reference instance: default use_icp = True, voxel size from the checkpoint
+  assert bool(ref['use_icp']) is True and float(ref['voxel_size']) == state['config']['voxel_size']
+  vs = float(ref['voxel_size'])
   T_o, taps = op.register(state, xyz0, xyz1, clip_weight_thresh=0.05, use_icp=True)
   assert taps['branch'] == 'procrustes'
-  printed = capsys.readouterr().out
-  assert f"=> Weighted sum {taps['wsum']:.2f} >=" in printed           # same gate value, same branch
-  call, = reference_dgr.icp_calls
-  assert call['max_dist'] == 2 * dgr.voxel_size and call['n_source'] == len(taps['coords0']) \
-      and call['n_target'] == len(taps['coords1'])
-  te, re = syn.rte_rre(call['init'], taps['T_refined'])                 # tap A: before ICP
+  assert f"=> Weighted sum {taps['wsum']:.2f} >=" in str(ref['printed'])       # same gate value, same branch
+  # what the reference handed to open3d's ICP
+  assert float(ref['icp_max_dist']) == 2 * vs and int(ref['icp_n_source']) == len(taps['coords0']) \
+      and int(ref['icp_n_target']) == len(taps['coords1'])
+  te, re = syn.rte_rre(ref['icp_init'], taps['T_refined'])                   # tap A: before ICP
   assert te <= 1e-3 and re <= 1e-3, (te, re, taps['refine'])
-  te, re = syn.rte_rre(T_ref, T_o)                                      # tap B: the literal return value
+  te, re = syn.rte_rre(ref['T'], T_o)                                        # tap B: the literal return value
   assert te <= 1e-3 and re <= 1e-3, (te, re, taps['icp'])
-  # stage taps through the reference's own methods
-  p0, c0, f0 = dgr.preprocess(xyz0)
-  assert np.array_equal(c0.numpy(), taps['coords0']) and np.array_equal(p0.numpy(), taps['xyz0'])
-  assert p0.dtype == torch.float32 and c0.dtype == torch.int32 and tuple(f0.shape) == (len(c0), 1)
-  with torch.no_grad():
-    F0 = dgr.fcgf_feature_extraction(f0, c0)
-  assert float((F0 - taps['feat0']).abs().max()) <= 1e-6
+  # stage taps of the reference's own methods: preprocess(xyz0) and fcgf_feature_extraction
+  assert str(ref['p0_dtype']) == 'torch.float32' and str(ref['c0_dtype']) == 'torch.int32'
+  assert sha(taps['coords0'].astype(np.int32)) == str(ref['sha_c0'])
+  assert sha(taps['xyz0'].astype(np.float32)) == str(ref['sha_p0'])
+  assert tuple(ref['f0_shape']) == (len(taps['coords0']), 1)
+  rows = ref['F0_rows']
+  assert float(np.abs(ref['F0'] - taps['feat0'].numpy()[rows]).max()) <= 1e-6
 
 
-def test_public_surface_matches_the_reference_class(reference_dgr):
+def test_public_surface_matches_the_reference_class(gold):
   """Same public methods with the same parameter names (and defaults where the reference has them) on
   deepglobalregistration_b200's DeepGlobalRegistration - the drop-in boundary of SURVEY.md 8(b)."""
   import inspect
 
   from deepglobalregistration_b200.core.deep_global_registration import DeepGlobalRegistration as Ours
-  ref_methods = {n: f for n, f in inspect.getmembers(reference_dgr, inspect.isfunction) if not n.startswith('_') or n == '__init__'}
+  ref_methods = json.loads(str(gold['surface']))
   assert set(ref_methods) == {'__init__', 'preprocess', 'fcgf_feature_extraction', 'fcgf_feature_matching',
                               'inlier_feature_generation', 'inlier_prediction', 'safeguard_registration', 'register'}
-  for name, f in ref_methods.items():
+  for name, want in ref_methods.items():
     ours = getattr(Ours, name, None)
     assert ours is not None, f'missing method {name}'
-    want = inspect.signature(f).parameters
     got = inspect.signature(ours).parameters
     public = [p for p in got if not p.startswith('_')]          # ours may add private keyword-only helpers
-    assert public == list(want), (name, public, list(want))
-    for p in want:
-      if want[p].default is not inspect.Parameter.empty and name != '__init__':
-        assert got[p].default == want[p].default, (name, p)
+    assert public == [p for p, _, _ in want], (name, public, want)
+    for p, has_default, default in want:
+      if has_default and name != '__init__':
+        assert repr(got[p].default) == default, (name, p)
   assert str(inspect.signature(Ours.__init__).parameters['device'].default) == 'cuda'
