@@ -21,6 +21,17 @@
 // product is off by at most 2^-10 |a||b| (+ accumulation slack), and d~2 by twice that.  The
 // true nearest neighbour j* satisfies d~2(j*) <= d2(j*) + E <= d2(j) + E <= d~2(j) + 2E for
 // every j, hence it is always among the candidates and the result equals the fp32 kernel's.
+//
+// FP16 operands (the default; DGR_KNN_TF32=1 selects the TF32 kernel): row i of F0 is multiplied by a power of
+// two s_i, all of F1 by one power of two t, each mapping the absolute maximum into [2^14, 2^15) (exact, and below
+// FP16's 65504), then rounded to FP16.  The epilogue multiplies the product by 1 / (s_i t) (exact), so estimates
+// stay in the original units.  In scaled units x' = s_i a, y' = t b, rounding gives |dx'_c| <= 2^-11 |x'_c| + 2^-25
+// (2^-11: FP16's unit roundoff for normal values, as TF32's; 2^-25: half the subnormal spacing 2^-24, which also
+// covers values that flush to zero).  Summing over c with Cauchy-Schwarz (sum |y'_c| <= sqrt(C) |y'|):
+//   |x'.y' - h(x').h(y')| <= (2^-10 + 2^-22) |x'||y'| + (2^-25 + 2^-36) sqrt(C) (|x'| + |y'|) + C 2^-50,
+// and divided by s_i t:  (2^-10 + 2^-22) |a||b| + 1.001 * 2^-25 sqrt(C) (|a| / t + |b| / s_i) + C 2^-50 / (s_i t).
+// The first term is the TF32 term; knn_error_bound_f16 adds the other two with |b| <= max_j |b_j|.
+#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -48,18 +59,25 @@ __global__ void row_norms_kernel(const float* __restrict__ f, int64_t n, int c, 
                                  unsigned* __restrict__ max_bits) {
   int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3;   // 8 lanes per row
   int sub = threadIdx.x & 7;
-  float s = 0.f;
+  float s = 0.f, amax = 0.f;
   if (row < n)
     for (int k = sub; k < c; k += 8) {
       float v = f[row * c + k];
       s = fmaf(v, v, s);
+      amax = fmaxf(amax, fabsf(v));
     }
   s += __shfl_xor_sync(0xffffffffu, s, 1);
   s += __shfl_xor_sync(0xffffffffu, s, 2);
   s += __shfl_xor_sync(0xffffffffu, s, 4);
+  amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, 1));
+  amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, 2));
+  amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, 4));
   if (row < n && sub == 0) {
     n2[row] = s;
-    if (max_bits != nullptr) atomicMax(max_bits, __float_as_uint(s));
+    if (max_bits != nullptr) {
+      atomicMax(max_bits, __float_as_uint(s));              // max |b|^2
+      atomicMax(max_bits + 1, __float_as_uint(amax));       // max |b_c|: the FP16 pre-filter's F1 scale
+    }
   }
 }
 
@@ -70,7 +88,7 @@ __global__ void knn_tc_init_kernel(unsigned* __restrict__ rowmin_bits, unsigned 
     rowmin_bits[i] = 0x7f800000u;
     packed[i] = ~0ull;
   }
-  if (i == 0) *max_bits = 0u;
+  if (i == 0) max_bits[0] = max_bits[1] = 0u;
 }
 
 // thr_i = m~_i + 2 E_i with E_i = 2 * (dot-product error bound).
@@ -82,13 +100,22 @@ __device__ __forceinline__ float knn_error_bound(float na, float nb, bool fine) 
   const float rel = fine ? 4e-6f : (0.0009765625f * 1.25f + 4e-5f);
   return rel * na * nb + 1e-6f * (na + nb) * (na + nb) + 1e-7f;
 }
+// FP16 pre-filter (see the header): the same relative term, plus the absolute error of values that land in the
+// FP16 subnormal range after scaling.  inv_sa, inv_sb: the (power-of-two) inverse scales of the row and of F1.
+__device__ __forceinline__ float knn_error_bound_f16(float na, float nb, float inv_sa, float inv_sb, int c) {
+  const float rc = sqrtf((float)c);
+  return knn_error_bound(na, nb, false) + 3.1e-8f * rc * (na * inv_sb + nb * inv_sa) +
+         (float)c * 1e-15f * inv_sa * inv_sb;
+}
+// inv_s0 != nullptr: FP16 pre-filter, per-row F0 scales inv_s0[i], F1 scale in nb2_max_bits[2]
 __global__ void knn_tc_threshold_kernel(const unsigned* __restrict__ rowmin_bits, const float* __restrict__ na2,
                                         const unsigned* __restrict__ nb2_max_bits, int64_t n0, int fine,
-                                        float* __restrict__ thr) {
+                                        const float* __restrict__ inv_s0, int c, float* __restrict__ thr) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n0) return;
   const float na = sqrtf(na2[i]), nb = sqrtf(__uint_as_float(*nb2_max_bits));
-  const float e = knn_error_bound(na, nb, fine != 0);
+  const float e = inv_s0 != nullptr ? knn_error_bound_f16(na, nb, inv_s0[i], __uint_as_float(nb2_max_bits[2]), c)
+                                    : knn_error_bound(na, nb, fine != 0);
   // stored in the epilogue's units: candidates satisfy (0.5 |b|^2 - a.b) <= thr'
   thr[i] = 0.5f * (__uint_as_float(rowmin_bits[i]) + 4.f * e - na2[i]);
 }
@@ -470,6 +497,253 @@ knn_tc_kernel(const float* __restrict__ f0, int n0, const float* __restrict__ f1
   }
 }
 
+// ================================ FP16 pre-filter (default) ==========================================
+// Operands are packed once per call into FP16 SWIZZLE_128B images (knn_pack_f16_kernel) and bulk-copied into a
+// ring of shared-memory stages by one thread; the grid is persistent: CTA b walks a contiguous range of
+// (row tile, column tile) work items, so every SM is busy to the end and TMEM is allocated once per CTA.
+// A CTA tile is 256 F0 rows (two M = 128 products sharing each B tile) x 128 F1 columns.
+constexpr int kRowsH = 256;
+constexpr int kColsH = 128;
+constexpr int kStagesH = 6;
+constexpr int kAImgH = kRowsH * 128;     // bytes: 128-byte rows, 64 halves (C = 32: halves 32..63 are zero)
+constexpr int kBImgH = kColsH * 128;
+constexpr int kThreadsH = (2 + kEpiWarps) * 32;     // producer warp, MMA warp, 8 epilogue warps
+
+struct KnnSharedH {
+  float nb[kStagesH][kColsH];            // 0.5 |b|^2 of the stage's columns (bulk-copied, first: 16-byte aligned)
+  unsigned long long full[kStagesH];     // B stage landed (tx bytes)
+  unsigned long long empty[kStagesH];    // B stage drained by the epilogue (its MMAs completed before that)
+  unsigned long long a_full[2], a_empty[2];
+  unsigned long long acc_full[2], acc_empty[2];
+  uint32_t tmem_base;
+};
+
+// One row per 8 threads, one 16-byte piece (8 halves) per thread, written at its swizzled position:
+// row r at r * 128 bytes, piece p at (p ^ (r & 7)) * 16 - the K-major SWIZZLE_128B image of umma_desc.
+// amax_bits == nullptr: per-row scale (F0), inv_scale[row] = 1 / scale; otherwise one scale for all rows
+// (F1), stored in inv_scale[0], and nbh[row] = 0.5 |b|^2 (+inf for padding rows: never a minimum).
+template <int C>
+__global__ void knn_pack_f16_kernel(const float* __restrict__ f, int64_t n, int64_t n_pad,
+                                    const unsigned* __restrict__ amax_bits, float* __restrict__ inv_scale,
+                                    const float* __restrict__ n2, float* __restrict__ nbh, uint4* __restrict__ img) {
+  const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
+  const int p = threadIdx.x & 7;
+  if (row >= n_pad) return;                 // n_pad % 4 == 0: whole warps leave
+  float x[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (row < n && p * 8 < C) {
+    const float4 u = __ldg(reinterpret_cast<const float4*>(f + row * C + p * 8));
+    const float4 v = __ldg(reinterpret_cast<const float4*>(f + row * C + p * 8 + 4));
+    x[0] = u.x; x[1] = u.y; x[2] = u.z; x[3] = u.w; x[4] = v.x; x[5] = v.y; x[6] = v.z; x[7] = v.w;
+  }
+  float am;
+  if (amax_bits == nullptr) {
+    am = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) am = fmaxf(am, fabsf(x[k]));
+    am = fmaxf(am, __shfl_xor_sync(0xffffffffu, am, 1));
+    am = fmaxf(am, __shfl_xor_sync(0xffffffffu, am, 2));
+    am = fmaxf(am, __shfl_xor_sync(0xffffffffu, am, 4));
+  } else {
+    am = __uint_as_float(*amax_bits);
+  }
+  const float sc = f16_scale_for(am);       // a power of two: x * sc is exact
+  uint32_t h[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const __half2 hh = __floats2half2_rn(x[2 * k] * sc, x[2 * k + 1] * sc);
+    h[k] = *reinterpret_cast<const uint32_t*>(&hh);
+  }
+  img[row * 8 + (p ^ (int)(row & 7))] = make_uint4(h[0], h[1], h[2], h[3]);
+  if (p == 0) {
+    if (amax_bits == nullptr) {
+      inv_scale[row] = 1.f / sc;
+    } else {
+      if (row == 0) inv_scale[0] = 1.f / sc;
+      nbh[row] = row < n ? 0.5f * n2[row] : __int_as_float(0x7f800000);
+    }
+  }
+}
+
+template <int C, int PASS>
+__global__ void __launch_bounds__(kThreadsH, 1)
+knn_f16_kernel(const unsigned char* __restrict__ a_img, const unsigned char* __restrict__ b_img,
+               const float* __restrict__ nbh, int n0, int n1, int n_ct, int64_t n_units,
+               const float* __restrict__ f0, const float* __restrict__ f1, const float* __restrict__ na2,
+               const float* __restrict__ inv_s0, const unsigned* __restrict__ max_bits,
+               unsigned* __restrict__ rowmin_bits, const float* __restrict__ thr,
+               unsigned long long* __restrict__ packed) {
+  extern __shared__ __align__(16) unsigned char smem_dyn[];
+  KnnSharedH& sh = *reinterpret_cast<KnnSharedH*>(smem_dyn);
+  unsigned char* a_buf = reinterpret_cast<unsigned char*>(
+      (reinterpret_cast<uintptr_t>(smem_dyn) + sizeof(KnnSharedH) + 1023) & ~(uintptr_t)1023);
+  unsigned char* b_buf = a_buf + 2 * kAImgH;
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  const int64_t u_begin = (int64_t)blockIdx.x * n_units / gridDim.x;
+  const int64_t u_end = (int64_t)(blockIdx.x + 1) * n_units / gridDim.x;
+
+  if (t == 0) {
+    for (int s = 0; s < kStagesH; ++s) {
+      mbar_init(smem_u32(&sh.full[s]), 1);
+      mbar_init(smem_u32(&sh.empty[s]), kEpiWarps * 32);
+    }
+    for (int b = 0; b < 2; ++b) {
+      mbar_init(smem_u32(&sh.a_full[b]), 1);
+      mbar_init(smem_u32(&sh.a_empty[b]), 1);
+      mbar_init(smem_u32(&sh.acc_full[b]), 1);
+      mbar_init(smem_u32(&sh.acc_empty[b]), kEpiWarps * 32);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
+                     smem_u32(&sh.tmem_base)),
+                 "r"(512u)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = sh.tmem_base;
+
+  if (warp == 0) {
+    // ================================ producer: one thread, bulk copies ===================
+    if (lane == 0) {
+      int it = 0, seg = 0;
+      for (int64_t u = u_begin; u < u_end; ++u, ++it) {
+        const int rt = (int)(u / n_ct), ct = (int)(u % n_ct);
+        if (u == u_begin || ct == 0) {       // a new row tile: the other A buffer, once its products are done
+          const int a = seg & 1;
+          mbar_wait(smem_u32(&sh.a_empty[a]), ((seg >> 1) & 1) ^ 1);
+          mbar_arrive_expect_tx(smem_u32(&sh.a_full[a]), kAImgH);
+          bulk_g2s(smem_u32(a_buf + a * kAImgH), a_img + (size_t)rt * kAImgH, kAImgH, smem_u32(&sh.a_full[a]));
+          ++seg;
+        }
+        const int s = it % kStagesH;
+        mbar_wait(smem_u32(&sh.empty[s]), ((it / kStagesH) & 1) ^ 1);
+        mbar_arrive_expect_tx(smem_u32(&sh.full[s]), kBImgH + kColsH * 4);
+        bulk_g2s(smem_u32(b_buf + s * kBImgH), b_img + (size_t)ct * kBImgH, kBImgH, smem_u32(&sh.full[s]));
+        bulk_g2s(smem_u32(sh.nb[s]), nbh + (size_t)ct * kColsH, kColsH * 4, smem_u32(&sh.full[s]));
+      }
+    }
+  } else if (warp == 1) {
+    // ================================ MMA issuer ==========================================
+    // D = F32, A = B = F16, both K-major, N = 128, M = 128; K = 16 halves (32 bytes) per instruction
+    const uint32_t idesc = (1u << 4) | ((uint32_t)(kColsH >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+    int it = 0, seg = 0, a = 0;
+    for (int64_t u = u_begin; u < u_end; ++u, ++it) {
+      const int ct = (int)(u % n_ct);
+      if (u == u_begin || ct == 0) {
+        a = seg & 1;
+        mbar_wait(smem_u32(&sh.a_full[a]), (seg >> 1) & 1);
+        ++seg;
+      }
+      const int b = it & 1, s = it % kStagesH;
+      mbar_wait(smem_u32(&sh.acc_empty[b]), ((it >> 1) & 1) ^ 1);
+      mbar_wait(smem_u32(&sh.full[s]), (it / kStagesH) & 1);
+      tc_fence_after();
+      if (lane == 0) {
+        const uint32_t a0 = smem_u32(a_buf + a * kAImgH), b0 = smem_u32(b_buf + s * kBImgH);
+        const uint32_t td = tmem_base + (uint32_t)b * 256;
+#pragma unroll
+        for (int ks = 0; ks < C / 16; ++ks) {
+          const uint64_t bd = umma_desc(b0 + ks * 32);
+          tc_mma_f16(td, umma_desc(a0 + ks * 32), bd, idesc, ks != 0);                      // rows 0..127
+          tc_mma_f16(td + 128, umma_desc(a0 + kAImgH / 2 + ks * 32), bd, idesc, ks != 0);   // rows 128..255
+        }
+        tc_commit(smem_u32(&sh.acc_full[b]));
+        if (u + 1 == u_end || ct == n_ct - 1) tc_commit(smem_u32(&sh.a_empty[a]));   // last tile of this A
+      }
+      __syncwarp();
+    }
+  } else {
+    // ================================ epilogue: thread = F0 row ===========================
+    const int lane_grp = warp & 3;                // TMEM lanes this warp may read
+    const int mh = (warp - 2) >> 2;               // 0: rows 0..127 of the tile, 1: rows 128..255
+    const int r = mh * 128 + lane_grp * 32 + lane;
+    const float pinf = __int_as_float(0x7f800000);
+    const float inv_s1 = __uint_as_float(max_bits[2]);
+    const float nb_max = sqrtf(__uint_as_float(max_bits[0]));
+    int gi = 0;
+    bool valid = false;
+    float inv = 0.f, th = -pinf, na2_i = 0.f, e4 = 0.f, rmin = pinf, best_s = pinf, best_d2 = pinf;
+    int best_j = 0x7fffffff;
+    int it = 0;
+    for (int64_t u = u_begin; u < u_end; ++u, ++it) {
+      const int rt = (int)(u / n_ct), ct = (int)(u % n_ct);
+      if (u == u_begin || ct == 0) {
+        gi = rt * kRowsH + r;
+        valid = gi < n0;
+        // D * inv is the product in the original units (inv: a power of two, the multiplication is exact)
+        inv = valid ? inv_s0[gi] * inv_s1 : 0.f;
+        rmin = pinf; best_s = pinf; best_d2 = pinf; best_j = 0x7fffffff;
+        if (PASS == 2) {
+          th = valid ? thr[gi] : -pinf;
+          // pass 2 tightens its bound with every exact distance it learns (see the TF32 kernel)
+          na2_i = valid ? na2[gi] : 0.f;
+          e4 = valid ? 4.f * knn_error_bound_f16(sqrtf(na2_i), nb_max, inv_s0[gi], inv_s1, C) : 0.f;
+        }
+      }
+      const int b = it & 1, s = it % kStagesH;
+      mbar_wait(smem_u32(&sh.acc_full[b]), (it >> 1) & 1);
+      mbar_wait(smem_u32(&sh.full[s]), (it / kStagesH) & 1);     // the norms' bulk copy
+      tc_fence_after();
+      const uint32_t taddr = tmem_base + (uint32_t)b * 256 + mh * 128 + ((uint32_t)(lane_grp * 32) << 16);
+      const float4* hb = reinterpret_cast<const float4*>(sh.nb[s]);
+      const int j0 = ct * kColsH;
+      uint32_t va[32], vb[32];
+      tc_ld32_issue(taddr, va);
+#pragma unroll
+      for (int cc = 0; cc < 4; ++cc) {
+        tc_ld_wait();
+        uint32_t(&cur)[32] = (cc & 1) ? vb : va;
+        uint32_t(&nxt)[32] = (cc & 1) ? va : vb;
+        if (cc < 3) tc_ld32_issue(taddr + (cc + 1) * 32, nxt);
+        const int jc = j0 + cc * 32;
+        if (jc < n1) {
+          float g[32];
+#pragma unroll
+          for (int q4 = 0; q4 < 8; ++q4) {
+            const float4 h4 = hb[cc * 8 + q4];
+            g[4 * q4 + 0] = fmaf(-__uint_as_float(cur[4 * q4 + 0]), inv, h4.x);
+            g[4 * q4 + 1] = fmaf(-__uint_as_float(cur[4 * q4 + 1]), inv, h4.y);
+            g[4 * q4 + 2] = fmaf(-__uint_as_float(cur[4 * q4 + 2]), inv, h4.z);
+            g[4 * q4 + 3] = fmaf(-__uint_as_float(cur[4 * q4 + 3]), inv, h4.w);
+          }
+          float cmin = pinf;
+#pragma unroll
+          for (int q = 0; q < 32; ++q) cmin = fminf(cmin, g[q]);
+          if (PASS == 1) {
+            rmin = fminf(rmin, cmin);
+          } else if (cmin <= th) {
+            const int nq = min(32, n1 - jc);
+#pragma unroll
+            for (int q = 0; q < 32; ++q) {
+              if (q < nq && g[q] <= th) {
+                knn_exact_candidate<C>(f0, f1, gi, jc + q, best_s, best_d2, best_j);
+                th = fminf(th, 0.5f * (best_d2 + e4 - na2_i));
+              }
+            }
+          }
+        }
+      }
+      tc_fence_before();
+      mbar_arrive(smem_u32(&sh.acc_empty[b]));
+      mbar_arrive(smem_u32(&sh.empty[s]));
+      if (valid && (u + 1 == u_end || ct == n_ct - 1)) {     // last column tile of this row tile in this CTA
+        if (PASS == 1) atomicMin(rowmin_bits + gi, __float_as_uint(fmaxf(fmaf(2.f, rmin, na2[gi]), 0.f)));
+        else if (best_j != 0x7fffffff)
+          atomicMin(packed + gi, ((unsigned long long)__float_as_uint(best_s) << 32) | (unsigned)best_j);
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+  }
+}
+
 __global__ void knn_tc_unpack_kernel(const unsigned long long* __restrict__ packed, int64_t n,
                                      int32_t* __restrict__ idx, float* __restrict__ dist) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -477,6 +751,58 @@ __global__ void knn_tc_unpack_kernel(const unsigned long long* __restrict__ pack
   unsigned long long p = packed[i];
   idx[i] = (int32_t)(p & 0xffffffffu);
   if (dist != nullptr) dist[i] = __uint_as_float((unsigned)(p >> 32));
+}
+
+// Workspace of dgr_knn_top1_tc, in floats.  The first 3 n0 + n1 + 8 are used by both pre-filters; the FP16 one
+// adds the operand images and per-row scales, each at a 256-byte boundary (bulk-copy sources need 16).
+struct KnnWs {
+  int64_t n0p, n1p, base, inv_s0, nbh, a_img, b_img, total;
+  KnnWs(int64_t n0, int64_t n1) {
+    n0p = (n0 + kRowsH - 1) / kRowsH * kRowsH;
+    n1p = (n1 + kColsH - 1) / kColsH * kColsH;
+    base = (3 * n0 + n1 + 8 + 63) / 64 * 64;
+    inv_s0 = base;
+    nbh = inv_s0 + n0p;
+    a_img = nbh + n1p;
+    b_img = a_img + n0p * 32;        // 128 bytes per row
+    total = b_img + n1p * 32;
+  }
+};
+
+int sm_count() {
+  int dev = 0, n = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+    return 148;
+  return n;
+}
+
+template <int C>
+int32_t launch_knn_f16(const float* f0, int64_t n0, const float* f1, int64_t n1, float* ws, unsigned* rowmin,
+                       float* thr, unsigned* max_bits, unsigned long long* packed, cudaStream_t st) {
+  const KnnWs w(n0, n1);
+  float* na2 = ws;
+  float* nb2 = ws + 3 * n0;
+  float* inv_s0 = ws + w.inv_s0;
+  float* nbh = ws + w.nbh;
+  unsigned char* a_img = reinterpret_cast<unsigned char*>(ws + w.a_img);
+  unsigned char* b_img = reinterpret_cast<unsigned char*>(ws + w.b_img);
+  knn_pack_f16_kernel<C><<<dgr_blocks(w.n0p * 8, 256), 256, 0, st>>>(f0, n0, w.n0p, nullptr, inv_s0, nullptr, nullptr,
+                                                                       reinterpret_cast<uint4*>(a_img));
+  knn_pack_f16_kernel<C><<<dgr_blocks(w.n1p * 8, 256), 256, 0, st>>>(
+      f1, n1, w.n1p, max_bits + 1, reinterpret_cast<float*>(max_bits + 2), nb2, nbh, reinterpret_cast<uint4*>(b_img));
+  const size_t smem = sizeof(KnnSharedH) + 1024 + 2 * (size_t)kAImgH + (size_t)kStagesH * kBImgH;
+  DGR_ENSURE_SMEM((knn_f16_kernel<C, 1>), smem);
+  DGR_ENSURE_SMEM((knn_f16_kernel<C, 2>), smem);
+  const int n_ct = (int)(w.n1p / kColsH);
+  const int64_t n_units = (w.n0p / kRowsH) * n_ct;
+  static const int n_sm = sm_count();
+  const int grid = (int)(n_units < n_sm ? n_units : n_sm);
+  knn_f16_kernel<C, 1><<<grid, kThreadsH, smem, st>>>(a_img, b_img, nbh, (int)n0, (int)n1, n_ct, n_units, f0, f1, na2,
+                                                      inv_s0, max_bits, rowmin, thr, packed);
+  knn_tc_threshold_kernel<<<dgr_blocks(n0, 256), 256, 0, st>>>(rowmin, na2, max_bits, n0, 0, inv_s0, C, thr);
+  knn_f16_kernel<C, 2><<<grid, kThreadsH, smem, st>>>(a_img, b_img, nbh, (int)n0, (int)n1, n_ct, n_units, f0, f1, na2,
+                                                      inv_s0, max_bits, rowmin, thr, packed);
+  return DGR_OK;
 }
 
 // single sweep (DGR_KNN_SWEEPS=1): no row-minimum pass, no threshold kernel
@@ -518,7 +844,8 @@ int32_t launch_knn_tc(const float* f0, int64_t n0, const float* f1, int64_t n1, 
   dim3 grid(row_tiles, splits);
   knn_tc_kernel<C, 1, kFine><<<grid, kThreadsK, smem, st>>>(f0, (int)n0, f1, (int)n1, na2, nb2, cols_per_split,
                                                             rowmin, thr, packed, max_bits);
-  knn_tc_threshold_kernel<<<dgr_blocks(n0, 256), 256, 0, st>>>(rowmin, na2, max_bits, n0, kFine ? 1 : 0, thr);
+  knn_tc_threshold_kernel<<<dgr_blocks(n0, 256), 256, 0, st>>>(rowmin, na2, max_bits, n0, kFine ? 1 : 0, nullptr,
+                                                               C, thr);
   knn_tc_kernel<C, 2, kFine><<<grid, kThreadsK, smem, st>>>(f0, (int)n0, f1, (int)n1, na2, nb2, cols_per_split,
                                                             rowmin, thr, packed, max_bits);
   return DGR_OK;
@@ -529,7 +856,7 @@ int32_t launch_knn_tc(const float* f0, int64_t n0, const float* f1, int64_t n1, 
 extern "C" {
 
 // floats of workspace dgr_knn_top1_tc needs
-int64_t dgr_knn_tc_ws_elems(int64_t n0, int64_t n1) { return 3 * n0 + n1 + 8; }
+int64_t dgr_knn_tc_ws_elems(int64_t n0, int64_t n1) { return KnnWs(n0, n1).total; }
 
 // 1 if the tensor-core pre-filter supports the channel count
 int32_t dgr_knn_tc_supported(int32_t c) { return (c == 32 || c == 64) ? 1 : 0; }
@@ -552,7 +879,20 @@ int32_t dgr_knn_top1_tc(const float* f0, int64_t n0, const float* f1, int64_t n1
   knn_tc_init_kernel<<<dgr_blocks(n0, 256), 256, 0, st>>>(rowmin, packed, n0, max_bits);
   row_norms_kernel<<<dgr_blocks(n0 * 8, 256), 256, 0, st>>>(f0, n0, c, na2, nullptr);
   row_norms_kernel<<<dgr_blocks(n1 * 8, 256), 256, 0, st>>>(f1, n1, c, nb2, max_bits);
-  // default: single TF32 product per term.  DGR_KNN_FINE=1 (c = 32 only): 3xTF32 products, a ~150x narrower
+  // default: the FP16 pre-filter.  DGR_KNN_TF32=1: the TF32 kernel it replaced, read on every call so that
+  // both can be timed in one process
+  const char* tf32_env = getenv("DGR_KNN_TF32");
+  const bool tf32 = tf32_env != nullptr && atoi(tf32_env) == 1;
+  if (!tf32) {
+    int32_t rc = (c == 32) ? launch_knn_f16<32>(f0, n0, f1, n1, ws, rowmin, thr, max_bits, packed, st)
+                           : launch_knn_f16<64>(f0, n0, f1, n1, ws, rowmin, thr, max_bits, packed, st);
+    if (rc != DGR_OK) return rc;
+    knn_tc_unpack_kernel<<<dgr_blocks(n0, 256), 256, 0, st>>>(packed, n0, idx, dist);
+    dgr_note_launches(9);
+    DGR_LAUNCH_CHECK();
+    return DGR_OK;
+  }
+  // DGR_KNN_TF32=1 only: DGR_KNN_FINE=1 (c = 32 only): 3xTF32 products, a ~150x narrower
   // candidate band, measured slower (the hi + lo tiles double the operand staging)
   static const bool coarse = getenv("DGR_KNN_FINE") == nullptr;        // A/B switch: 3xTF32 pre-filter (slower)
   // DGR_KNN_SWEEPS=1: the single-sweep variant (running bound + candidate buffer)

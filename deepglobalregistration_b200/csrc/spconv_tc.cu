@@ -86,15 +86,6 @@ __device__ __forceinline__ void split_store_f16(float4 a, float4 b, float sx, un
   *reinterpret_cast<uint4*>(hi_tile + off) = make_uint4(h[0], h[1], h[2], h[3]);
   *reinterpret_cast<uint4*>(lo_tile + off) = make_uint4(l[0], l[1], l[2], l[3]);
 }
-// power of two that maps `amax` into [2^14, 2^15); 1 for amax == 0 / non-finite
-__device__ __forceinline__ float f16_scale_for(float amax) {
-  const uint32_t b = __float_as_uint(amax);
-  const int e = (int)((b >> 23) & 255u);
-  if (e == 0 || e == 255) return 1.f;
-  int se = 14 - (e - 127) + 127;
-  se = se < 1 ? 1 : (se > 254 ? 254 : se);
-  return __uint_as_float((uint32_t)se << 23);
-}
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
@@ -119,19 +110,6 @@ __device__ __forceinline__ void tc_commit_multicast(uint32_t bar, uint16_t mask)
       "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
       "h"(mask)
       : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// 1-D bulk copy global -> shared (TMA engine), completion signalled on an mbarrier
-__device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   dst_smem),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
 }
 
 

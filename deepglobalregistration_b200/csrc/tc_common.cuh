@@ -29,6 +29,19 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   while (!mbar_try_wait(bar, parity)) {
   }
 }
+__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
+  asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+// 1-D bulk copy global -> shared (TMA engine), completion signalled on an mbarrier
+__device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                   dst_smem),
+               "l"(src), "r"(bytes), "r"(bar)
+               : "memory");
+}
 __device__ __forceinline__ void fence_proxy_async() {
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
@@ -48,6 +61,15 @@ __device__ __forceinline__ void tc_mma_tf32(uint32_t tmem_d, uint64_t adesc, uin
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                           uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -108,6 +130,16 @@ __device__ __forceinline__ float tf32_round(float x) {
   uint32_t r;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
   return __uint_as_float(r);
+}
+
+// power of two that maps `amax` into [2^14, 2^15); 1 for amax == 0 / non-finite
+__device__ __forceinline__ float f16_scale_for(float amax) {
+  const uint32_t b = __float_as_uint(amax);
+  const int e = (int)((b >> 23) & 255u);
+  if (e == 0 || e == 255) return 1.f;
+  int se = 14 - (e - 127) + 127;
+  se = se < 1 ? 1 : (se > 254 ? 254 : se);
+  return __uint_as_float((uint32_t)se << 23);
 }
 
 // K-major SWIZZLE_128B operand descriptor: 8-row groups of 128-byte rows, 1024 bytes apart.
